@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W              # our arm (one rank per GPU; torchrun for N > 1)
   python bench.py --impl reference --gpus N --steps K --warmup W   # the reference's own CPU classes (oracle/_ref) on host cores
+  python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR  # also writes what the last timed rollout returned, DIR/<name>.npy
 
 A "step" is ONE ROLLOUT: `batch` prompts per rank x 30 denoise steps x (2 transformer forwards with CFG) + the fused
 Euler/SDE + log-prob step, synthetic inputs of the BASELINE shape, random-init weights of the SD3.5-medium architecture
@@ -66,6 +67,10 @@ def parse():
     ap.add_argument("--num-sde-steps", type=int, default=1)
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--skip-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed rollouts, write what the last one returned to its caller (rank 0: kept latents, log-probs, final "
+                         "latents and timesteps of the batch) as DIR/<name>.npy in float32, at most 64 MB in all; the inputs are seeded, so "
+                         "two builds run with the same arguments can be compared output for output")
     ap.add_argument("--config", default="sd35", choices=["sd35", "flux1", "wan21", "qwen_image"],
                     help="BASELINE.json config: sd35 = C2 (the metric's, default); flux1 / wan21 / qwen_image = configs 3-5, each through its own "
                          "bench tool under tools/ with the same line contract (examples/grpo/*/{flux1/default,wan21/t2v,qwen_image/default}.yaml)")
@@ -131,6 +136,29 @@ def flops_per_latent(cfg, ni, nt, T, cfg_on):
     from flow_factory_b200.synth import flops_per_forward
     lin, att = flops_per_forward(cfg, ni, nt)
     return (lin + att) * T * (2 if cfg_on else 1)
+
+
+DUMP_LIMIT_BYTES = 63_000_000      # 64 MB with room for the .npy headers
+
+
+def dump_outputs(directory: str, arrays) -> None:
+    """Write `arrays` (name -> tensor; None entries skipped) as DIR/<name>.npy, float64 kept, everything else as float32.  When they would
+    take more than DUMP_LIMIT_BYTES in all, every array above 1 MB is cut to the same fraction of its flattened elements, at positions drawn
+    from a fixed seed, so that two runs with the same arguments write the same positions."""
+    import numpy as np
+    arrays = {k: v.detach() for k, v in arrays.items() if v is not None}
+    size = lambda v: v.numel() * (8 if v.dtype == torch.float64 else 4)
+    large = {k for k, v in arrays.items() if size(v) > 1_000_000}
+    small_bytes = sum(size(v) for k, v in arrays.items() if k not in large)
+    large_bytes = sum(size(arrays[k]) for k in large)
+    os.makedirs(directory, exist_ok=True)
+    for name, v in arrays.items():
+        if name in large and small_bytes + large_bytes > DUMP_LIMIT_BYTES:
+            keep = v.numel() * (DUMP_LIMIT_BYTES - small_bytes) // large_bytes
+            idx = torch.randint(v.numel(), (keep,), generator=torch.Generator().manual_seed(0)).sort().values
+            v = v.flatten()[idx.to(v.device)]
+        v = v.cpu().double() if v.dtype == torch.float64 else v.cpu().float()
+        np.save(os.path.join(directory, name + ".npy"), v.numpy())
 
 
 # ------------------------------------------------------------------------------------------------ CPU baseline: the reference's own code
@@ -329,6 +357,7 @@ def run_b200(args):
     dev = torch.device("cuda", local)
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
+    torch.manual_seed(1 + rank)     # the adapter draws each rollout's noise seed from the global generator: same arguments, same noise
     cfg = sd35_medium()
     T, B = args.num_inference_steps, args.batch
     lat_h, lat_w = args.height // 8, args.width // 8
@@ -375,7 +404,7 @@ def run_b200(args):
     t_wall = time.perf_counter()
     e0.record()
     for _ in range(args.steps):
-        rollout_device()
+        last = rollout_device()
     e1.record()
     barrier()
     wall = time.perf_counter() - t_wall
@@ -385,6 +414,10 @@ def run_b200(args):
     ms_total = float(ms)
     clk = clocks.stop() if rank == 0 else None
     value = world * B * args.steps / (ms_total / 1e3)
+    if args.dump_outputs and rank == 0:       # now: the legs below reuse the engine's output buffers
+        stack = lambda name: None if getattr(last[0], name) is None else torch.stack([getattr(x, name) for x in last])
+        dump_outputs(args.dump_outputs, {"all_latents": stack("all_latents"), "log_probs": stack("log_probs"),
+                                         "final_latents": stack("final_latents"), "timesteps": last[0].timesteps})
 
     # ---------------- the same rollout with the WHOLE SDE window noisy (num_sde_steps = T - 1 = 29: noise + log-prob on every step but the
     # last; SURVEY 8d asks for {1, 29}) - one warm-up (the graph is re-used, only the step coefficients change), then timed ----------------
@@ -526,6 +559,8 @@ def run_other_config(args):
 
 def main():
     args = parse()
+    if args.dump_outputs and (args.impl != "b200" or args.config != "sd35"):
+        raise SystemExit("--dump-outputs is implemented for the engine arm of the sd35 config")
     if args.impl == "reference":
         run_reference(args)
     else:
