@@ -241,7 +241,7 @@ def flux_forward(w: Dict[str, torch.Tensor], cfg: FluxConfig, hidden_states: tor
         temb = temb + _mlp("time_text_embed.guidance_embedder", timestep_embedding(guidance, 256).to(dtype=pooled_projections.dtype))
     temb = temb + _mlp("time_text_embed.text_embedder", pooled_projections)
     ehs = _linear(w, "context_embedder", encoder_hidden_states)
-    cos, sin = rope_tables(torch.cat((txt_ids, img_ids), dim=0), cfg.axes_dims_rope)
+    cos, sin = (t.to(hs.device) for t in rope_tables(torch.cat((txt_ids, img_ids), dim=0), cfg.axes_dims_rope))
     if return_intermediates:
         inter["temb"], inter["hs0"], inter["ehs0"], inter["cos"], inter["sin"] = temb, hs, ehs, cos, sin
     for i in range(cfg.num_layers):

@@ -176,11 +176,11 @@ def qwen_forward(w: Dict[str, torch.Tensor], cfg: QwenImageConfig, hidden_states
     tproj = _timesteps_scaled(timestep)
     temb = _linear(w, "time_text_embed.timestep_embedder.linear_2",
                    F.silu(_linear(w, "time_text_embed.timestep_embedder.linear_1", tproj.to(dtype=hs.dtype))))
-    vid_freqs, txt_freqs = qwen_rope(*img_shape, encoder_hidden_states.shape[1], cfg.axes_dims_rope)
+    vid_freqs, txt_freqs = (f.to(hs.device) for f in qwen_rope(*img_shape, encoder_hidden_states.shape[1], cfg.axes_dims_rope))
     mask = None
     if encoder_hidden_states_mask is not None:
-        m = encoder_hidden_states_mask.to(torch.bool)
-        mask = torch.cat([m, torch.ones((hs.shape[0], hs.shape[1]), dtype=torch.bool)], dim=1)[:, None, None, :]
+        m = encoder_hidden_states_mask.to(device=hs.device, dtype=torch.bool)
+        mask = torch.cat([m, torch.ones((hs.shape[0], hs.shape[1]), dtype=torch.bool, device=hs.device)], dim=1)[:, None, None, :]
     for i in range(cfg.num_layers):
         ehs, hs = _qwen_block(w, i, cfg, hs, ehs, temb, vid_freqs, txt_freqs, mask)
     emb = _linear(w, "norm_out.linear", F.silu(temb).to(hs.dtype))
@@ -192,7 +192,7 @@ def qwen_forward(w: Dict[str, torch.Tensor], cfg: QwenImageConfig, hidden_states
 def _timesteps_scaled(timesteps: torch.Tensor, dim: int = 256, scale: float = 1000.0) -> torch.Tensor:
     """get_timestep_embedding(flip_sin_to_cos=True, downscale_freq_shift=0, scale=1000) (DF/models/embeddings.py:26-77)."""
     half = dim // 2
-    exponent = -math.log(10000) * torch.arange(0, half, dtype=torch.float32) / half
+    exponent = -math.log(10000) * torch.arange(0, half, dtype=torch.float32, device=timesteps.device) / half
     emb = torch.exp(exponent)
     emb = timesteps[:, None].float() * emb[None, :]
     emb = scale * emb

@@ -1,4 +1,5 @@
 """Helpers for the -m gpu parity tests: call the C ABI through ctypes on torch-owned device memory."""
+import contextlib
 import ctypes as C
 import json
 import os
@@ -45,6 +46,41 @@ def err_report(got: torch.Tensor, ref: torch.Tensor, tag: str):
         rep["got_00"] = g[:2, :8].tolist()
         rep["ref_00"] = r[:2, :8].tolist()
     return rep
+
+
+def chunked_sdpa(q, k, v, attn_mask=None, dropout_p=0.0, is_causal=False, scale=None):
+    """fp32 softmax(q k^T * scale) v over [B, H, S, d], a block of query rows at a time so that no score matrix exceeds ~2 GB
+    (torch's math backend would hold all B x H x Sq x Skv scores; Wan2.1 at 20 280 tokens needs 40 GB of them).
+    `attn_mask`: bool, True = attend (the Qwen-Image key-padding mask)."""
+    assert dropout_p == 0.0 and not is_causal and q.dtype == torch.float32, (dropout_p, is_causal, q.dtype)
+    scale = q.shape[-1] ** -0.5 if scale is None else scale
+    B, H, Sq, _ = q.shape
+    step = max(1, (1 << 29) // (B * H * k.shape[-2]))
+    kt = k.transpose(-1, -2)
+    out = torch.empty(*q.shape[:-1], v.shape[-1], dtype=q.dtype, device=q.device)
+    for s in range(0, Sq, step):
+        sc = torch.matmul(q[..., s:s + step, :], kt) * scale
+        if attn_mask is not None:
+            sc = sc.masked_fill(~attn_mask, float("-inf"))
+        out[..., s:s + step, :] = torch.matmul(sc.softmax(-1), v)
+    return out
+
+
+@contextlib.contextmanager
+def ieee_fp32():
+    """The fp32 truth of a parity test in IEEE fp32: TF32 off for matmul and cuDNN (torch enables it for cuDNN convolutions by
+    default), and scaled_dot_product_attention - which the oracles call through torch.nn.functional - replaced by chunked_sdpa.
+    Everything is restored on exit; bf16-autocast references must run outside this context."""
+    import torch.nn.functional as F
+    saved = torch.backends.cuda.matmul.allow_tf32, torch.backends.cudnn.allow_tf32, F.scaled_dot_product_attention
+    torch.backends.cuda.matmul.allow_tf32 = False
+    torch.backends.cudnn.allow_tf32 = False
+    F.scaled_dot_product_attention = chunked_sdpa
+    try:
+        with torch.no_grad():
+            yield
+    finally:
+        torch.backends.cuda.matmul.allow_tf32, torch.backends.cudnn.allow_tf32, F.scaled_dot_product_attention = saved
 
 
 from flow_factory_b200.ops import linear  # noqa: E402,F401

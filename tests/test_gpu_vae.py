@@ -11,6 +11,7 @@ pytestmark = pytest.mark.gpu
 
 from flow_factory_b200 import vae as V          # noqa: E402
 from oracle import vae_oracle as VO              # noqa: E402  (the checker)
+from tests.gpu_util import ieee_fp32, record     # noqa: E402
 
 DEV = "cuda"
 
@@ -29,7 +30,8 @@ def test_conv3x3_matches_torch(B, H, W, cin, cout, residual):
     b = (torch.randn(cout, generator=g, device=DEV) * 0.1).bfloat16()
     res = torch.randn(B, H, W, cout, generator=g, device=DEV).bfloat16() if residual else None
     out = V.conv2d_nhwc(x, w, b, res)
-    ref = F.conv2d(x.permute(0, 3, 1, 2).float(), w.float(), b.float(), padding=1).permute(0, 2, 3, 1)
+    with ieee_fp32():
+        ref = F.conv2d(x.permute(0, 3, 1, 2).float(), w.float(), b.float(), padding=1).permute(0, 2, 3, 1)
     ref = ref.bfloat16().float()
     if residual:
         ref = (ref + res.float())
@@ -46,7 +48,8 @@ def test_conv1x1_matches_linear(rows, cin, cout):
     w = (torch.randn(cout, cin, generator=g, device=DEV) / cin ** 0.5).bfloat16()
     b = (torch.randn(cout, generator=g, device=DEV) * 0.1).bfloat16()
     out = V.conv2d_nhwc(x, w, b)
-    ref = F.linear(x.float(), w.float(), b.float())
+    with ieee_fp32():
+        ref = F.linear(x.float(), w.float(), b.float())
     assert _rel(out, ref) < 6e-3
 
 
@@ -57,7 +60,8 @@ def test_group_norm_matches_torch(B, P, C, groups, silu):
     gamma = (1 + 0.1 * torch.randn(C, generator=g, device=DEV)).bfloat16()
     beta = (0.1 * torch.randn(C, generator=g, device=DEV)).bfloat16()
     out = V.group_norm_nhwc(x, gamma, beta, groups, 1e-6, silu)
-    ref = F.group_norm(x.float().permute(0, 2, 1), groups, gamma.float(), beta.float(), 1e-6).permute(0, 2, 1)
+    with ieee_fp32():
+        ref = F.group_norm(x.float().permute(0, 2, 1), groups, gamma.float(), beta.float(), 1e-6).permute(0, 2, 1)
     if silu:
         ref = F.silu(ref)
     torch.testing.assert_close(out.float(), ref.bfloat16().float(), rtol=1.6e-2, atol=1e-2)
@@ -73,8 +77,9 @@ def _decode_case(ocfg, lat, batch, seed):
     torch.cuda.synchronize()
     wd = {k: v.to(DEV) for k, v in w32.items()}
     lat16 = lat.half().float().to(DEV)
+    with ieee_fp32():
+        truth = VO.vae_decode(wd, ocfg, lat16)                                   # IEEE fp32
     with torch.no_grad():
-        truth = VO.vae_decode(wd, ocfg, lat16)                                   # fp32
         with torch.autocast("cuda", dtype=torch.bfloat16):
             ref16 = VO.vae_decode({k: v.bfloat16() for k, v in wd.items()}, ocfg, lat16.bfloat16())   # the reference's bf16 autocast numerics
     return img, truth, ref16, dec
@@ -103,7 +108,8 @@ def test_decode_matches_oracle(name, ocfg, shape, batch):
     img, truth, ref16, dec = _decode_case(ocfg, lat, batch, seed=7)
     assert torch.isfinite(img.float()).all()
     e_eng, e_ref = _rel(img, truth), _rel(ref16, truth)
-    assert e_eng <= 1.3 * e_ref + 5e-4, (e_eng, e_ref)       # as close to fp32 as the reference's own bf16 path
+    record("parity_measured.jsonl", dict(tag=f"vae_decode_{name}", e_engine=e_eng, e_ref_bf16=e_ref, ratio=e_eng / e_ref))
+    assert e_eng <= 1.3 * e_ref + 5e-4, (e_eng, e_ref)       # as close to fp32 as the reference's own bf16 path; measured on B200: 0.89, 0.90 x
     assert _rel(img, ref16) < 4 * e_ref + 2e-3
     assert torch.allclose(V.postprocess_pt(img).float(), (img.float() / 2 + 0.5).clamp(0, 1), atol=1e-2)
 
@@ -114,5 +120,6 @@ def test_decode_sd35_geometry_smoke():
     lat = torch.randn(1, 16, 64, 64, generator=torch.Generator().manual_seed(9))
     img, truth, ref16, dec = _decode_case(ocfg, lat, 1, seed=11)
     e_eng, e_ref = _rel(img, truth), _rel(ref16, truth)
-    assert e_eng <= 1.3 * e_ref + 5e-4, (e_eng, e_ref)
+    record("parity_measured.jsonl", dict(tag="vae_decode_sd35_512", e_engine=e_eng, e_ref_bf16=e_ref, ratio=e_eng / e_ref))
+    assert e_eng <= 1.3 * e_ref + 5e-4, (e_eng, e_ref)          # measured on B200 against the IEEE fp32 truth: 0.87 x
     assert dec.workspace_bytes() < 8 << 30
